@@ -2,6 +2,7 @@
 
     python bench.py [--gpus N --steps K --warmup W] [--impl reference]
                     [--mode infer|train] [--model yolov6s] [--batch 32] [--size 640] [--no-extra]
+                    [--dump-outputs DIR]
 
 The default run prints ONE JSON line whose headline (`value`, `e2e`, `roofline`) is BASELINE.json's config 2 and which
 also carries, under `modes`, the fp32-equivalent (bf16x3) precision mode with the measured bf16-vs-fp32 deviation on the
@@ -19,6 +20,12 @@ e2e = same metric through the public API from pinned HOST uint8 images incl. H2D
 detections; roofline = algorithmic conv FLOPs / measured conv-kernel time vs the measured bf16 peak;
 cpu_baseline = the oracle (CPU restatement of the reference path) on a bounded sample of the workload.
 `--impl reference` times that CPU path alone with all host threads.
+
+`--dump-outputs DIR` writes, after the timed steps of the headline, what its last step computed as .npy files (rank 0):
+inference: `detections.npy` float32 [n, 6] -- the per-image (x1, y1, x2, y2, conf, cls) rows `non_max_suppression` returns,
+concatenated in image order -- and `counts.npy` float64 [batch], the rows per image; with CUDA graphs the last step's NMS
+branch post-processes the batch before it (DetectStream), and those are its detections.  Training: `loss.npy` float64 [8],
+what `TrainStep.run` returns.  Weights and inputs are seeded, so the same arguments give the same inputs on every run.
 """
 import argparse
 import json
@@ -199,8 +206,26 @@ def load_peaks():
     return {}
 
 
-def bench_infer(model_name, B, S, steps, warmup, rank, world, dev, precision="bf16", e2e=True, roofline=True, graph=True):
-    """Forward + decode + batched NMS of `model_name` on B images of S x S per GPU.  Returns a dict of measurements."""
+def caller_detections(out, count, overflow):
+    """The detections `non_max_suppression` would return for nms_batched's (out, count, overflow), as numpy arrays."""
+    if int(overflow.item()):
+        raise RuntimeError("non_max_suppression: more than 65536 near-identical candidate scores in one image")
+    n = count.tolist()
+    rows = torch.cat([out[b, :k] for b, k in enumerate(n)])
+    return {"detections": rows.float().cpu().numpy(), "counts": torch.tensor(n, dtype=torch.float64).numpy()}
+
+
+def dump_outputs(path, arrays):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
+def bench_infer(model_name, B, S, steps, warmup, rank, world, dev, precision="bf16", e2e=True, roofline=True, graph=True,
+                keep_outputs=False):
+    """Forward + decode + batched NMS of `model_name` on B images of S x S per GPU.  Returns a dict of measurements
+    (with keep_outputs, `_outputs`: the detections of the last timed step)."""
     from yolov6_b200.model import build_model
     from yolov6_b200.nms import nms_batched
     from yolov6_b200.pipeline import DetectFarm
@@ -226,12 +251,22 @@ def bench_infer(model_name, B, S, steps, warmup, rank, world, dev, precision="bf
         def step_device(i):
             stream_dev.launch()
     else:
+        last = {}
+
         def step_device(i):
             pred = eng.forward(dev_f32[i & 1])
-            return nms_batched(pred, **NMS_KW)
+            last["nms"] = nms_batched(pred, **NMS_KW)
     with torch.no_grad():
         ms_dev = timed(step_device, steps, warmup, world, dev, farm=stream_dev if graph else None)
         out["ms_per_step"] = ms_dev
+        if keep_outputs:
+            if graph:
+                lane = stream_dev.lanes[(stream_dev.n - 1) % len(stream_dev.lanes)]
+                res = lane.dev_step[1 - ((lane.steps - 1) & 1)]     # the NMS branch of the lane's last graph
+            else:
+                o, c, _, ov = last["nms"]
+                res = (o, c, ov)
+            out["_outputs"] = caller_detections(*res)
         out["value"] = world * B / (ms_dev * 1e-3)
         if e2e:
             if graph:
@@ -289,7 +324,7 @@ TRAIN_LOSS = {"yolov6n": dict(use_dfl=False, reg_max=0, iou_type="siou"), "yolov
               "yolov6m": dict(use_dfl=True, reg_max=16, iou_type="giou"), "yolov6l6": dict(use_dfl=True, reg_max=16, iou_type="giou")}
 
 
-def bench_train(model_name, B, S, steps, warmup, rank, world, dev, graph=True):
+def bench_train(model_name, B, S, steps, warmup, rank, world, dev, graph=True, keep_outputs=False):
     """One training step of `model_name` on B images per GPU (BASELINE.json config 3 / 4): train-form forward, TAL
     assignment, VFL + IoU (+ DFL) loss, backward, gradient all-reduce over NCCL when world > 1; the optimizer (fused SGD +
     EMA) is timed separately and inside the end-to-end number."""
@@ -325,6 +360,7 @@ def bench_train(model_name, B, S, steps, warmup, rank, world, dev, graph=True):
         loss_host.copy_(out, non_blocking=True)           # D2H: loss / loss items
 
     ms_dev = timed(step_device, steps, warmup, world, dev)
+    outputs = {"loss": step.state["out"].double().cpu().numpy()}
     first_loss = [float(v) for v in step.state["out"][:4].tolist()]
     ar_ms = step.sync.last_ms() if step.sync is not None else 0.0
     ms_opt = timed(step_opt, steps, 1, world, dev)
@@ -338,7 +374,7 @@ def bench_train(model_name, B, S, steps, warmup, rank, world, dev, graph=True):
     gflop_img = 3.0 * GFLOP_PER_IMG[model_name] * (S / (1280.0 if model_name == "yolov6l6" else 640.0)) ** 2
     achieved = gflop_img * 1e9 * B / (ms_dev * 1e-3) / 1e12
     peak = float(peaks.get("bf16_tflops_sustained", 1400.0))
-    return {"model": model_name, "batch_per_gpu": B, "size": S, "value": world * B / (ms_dev * 1e-3), "unit": "images/s",
+    res = {"model": model_name, "batch_per_gpu": B, "size": S, "value": world * B / (ms_dev * 1e-3), "unit": "images/s",
             "ms_per_step": ms_dev, "step": "train-form forward + TAL + VFL/GIoU" + ("/DFL" if TRAIN_LOSS[model_name]["use_dfl"] else "") +
             " loss + backward" + (" + gradient all-reduce" if world > 1 else ""),
             "optimizer_ms": ms_opt, "optimizer": "fused SGD-nesterov + weight decay + EMA, one kernel (yv6_sgd_ema_step)",
@@ -352,6 +388,9 @@ def bench_train(model_name, B, S, steps, warmup, rank, world, dev, graph=True):
             "roofline": {"bound": "tensor", "achieved": achieved, "peak": peak, "unit": "TFLOP/s", "frac": achieved / peak,
                          "algorithmic_gflop_per_img": gflop_img,
                          "note": "3 x the deploy-form forward FLOPs (fwd + dgrad + wgrad), SURVEY.md 8d; the train form executes ~9 % more"}}
+    if keep_outputs:
+        res["_outputs"] = outputs
+    return res
 
 
 def free_cuda():
@@ -377,7 +416,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the fp32-mode leg and the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline computed to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl ours)")
     if args.size is None:
         args.size = 1280 if args.model == "yolov6l6" else 640
     if args.batch is None:
@@ -401,7 +446,10 @@ def main():
     short = max(5, min(args.steps, 20))
 
     if args.mode == "train":
-        tr = bench_train(args.model, B, S, args.steps, W, rank, world, dev, graph=use_graph)
+        tr = bench_train(args.model, B, S, args.steps, W, rank, world, dev, graph=use_graph, keep_outputs=bool(args.dump_outputs))
+        outputs = tr.pop("_outputs", None)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, outputs)
         sampler.stop_flag = True
         sampler.join(timeout=2)
         if rank == 0:
@@ -423,8 +471,11 @@ def main():
         return
 
     # ---------------------------------------------------------------- inference headline (BASELINE.json config 2)
-    main_r = bench_infer(args.model, B, S, args.steps, W, rank, world, dev, precision=args.precision, graph=use_graph)
+    main_r = bench_infer(args.model, B, S, args.steps, W, rank, world, dev, precision=args.precision, graph=use_graph,
+                         keep_outputs=bool(args.dump_outputs))
     model, x0 = main_r.pop("_model"), main_r.pop("_input")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, main_r.pop("_outputs"))
     modes, check, extra = {}, None, {}
     if not args.no_extra:
         check = precision_check(model, x0, dev)
